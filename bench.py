@@ -31,16 +31,23 @@ One JSON line on rank 0:
   multirank_parity (N > 1) per-rank loss / grad-norm / d temperature of a tiny sharded step against
                the oracle's restatement of the reference's per-rank contract (distributed.py:41-56)
 `--impl reference` times the reference's own CPU implementation of the same model on the host.
+`--dump-outputs DIR` writes what the last device-resident timed step returned to its caller: the loss
+and every parameter gradient, as DIR/loss.npy and DIR/grad.<parameter name>.npy (float32; a fixed,
+seeded sample of each large gradient, at most 64 MB in all).  Same arguments give the same inputs, so
+the dumps of two builds can be compared array by array.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
+import math
 import os
 import subprocess
 import sys
 import threading
 import time
+import zlib
 from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
@@ -93,7 +100,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg2 / cfg4 / cfg5 side measurements")
     ap.add_argument("--no-parity", action="store_true", help="skip the N>1 per-rank parity check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and the parameter gradients of the last timed step to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU step (--impl ours)")
     a.retain = a.retain if a.retain == "auto" else int(a.retain)
     d = DEFAULTS[a.workload]
     if a.batch is None:
@@ -123,7 +136,6 @@ def _reference_module(model_cfg, loss_kw, patch_dropout, device="cpu"):
     to None when oracle/_ref was never built (then the oracle port is timed instead)."""
     try:
         from oracle import build_ref
-        build_ref.build()                       # no-op when present / when /root/reference is absent
         x_clip = build_ref.import_reference()
     except Exception:
         return None
@@ -222,6 +234,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--query-gpu={self.QUERY}", "--format=csv,noheader,nounits",
                  "-lms", "100", "-i", str(self.index)], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.kill)     # never outlive the benchmark, even when it fails
             threading.Thread(target=self._pump, daemon=True).start()
         except Exception:
             self.proc = None
@@ -335,6 +348,30 @@ class Runner:
             self.grad_sync.remove()
         self.clip = self.params = self.text = self.image = self.host = None
         self.torch.cuda.empty_cache()
+
+
+DUMP_VALUES = 8 * 2**20     # sampled gradient values, float32: 32 MB, plus <= 4096 per tensor (64 MB cap)
+
+
+def step_outputs(loss, clip):
+    """-> {name: float32 numpy array} of what one step hands its caller: the loss and each parameter's
+    gradient.  A gradient larger than its share of DUMP_VALUES is sampled at sorted positions drawn
+    without replacement from a generator seeded by the parameter name, the same positions in every run."""
+    import numpy as np
+    import torch
+    grads = [(n, p.grad) for n, p in clip.named_parameters() if p.grad is not None]
+    frac = min(1.0, DUMP_VALUES / sum(g.numel() for _, g in grads))
+    out = {"loss": np.asarray(loss.item(), dtype=np.float32)}
+    for name, g in grads:
+        flat = g.detach().float().reshape(-1)
+        k = min(flat.numel(), max(4096, math.ceil(flat.numel() * frac)))
+        if k < flat.numel():
+            gen = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randperm(flat.numel(), generator=gen)[:k].sort().values
+            flat = flat[idx.to(flat.device)]
+        out[f"grad.{name}"] = flat.cpu().numpy()
+    assert sum(a.nbytes for a in out.values()) <= 64 * 2**20
+    return out
 
 
 def multirank_parity(dev, rank, world):
@@ -503,6 +540,13 @@ def main():
     peak_mem = torch.cuda.max_memory_allocated(dev)
     clocks = sampler.stop() if rank == 0 else None
     note(f"device-resident timing done: {ms_dev / args.steps:.1f} ms/step")
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for name, arr in step_outputs(loss, run.clip).items():
+            np.save(out_dir / f"{name}.npy", arr)
+        note(f"outputs of the last timed step written to {out_dir}")
 
     # ---- (2) end-to-end: pinned host -> device copy of every step's batch (side stream, double
     #          buffered) + loss read-back, all inside the timed region

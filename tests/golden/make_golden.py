@@ -12,9 +12,12 @@ the SURVEY 4 seed protocol) and refuses to write fixtures if they disagree.
 """
 from __future__ import annotations
 
+import inspect
 import json
 import os
+import random
 import sys
+import zlib
 from pathlib import Path
 
 import torch
@@ -100,7 +103,9 @@ def build_reference(x_clip, cfg_kwargs, patch_dropout, state):
     return clip
 
 
-def run_case(x_clip, name, cfg_kwargs, batch, pad_fraction, patch_dropout):
+def run_case(x_clip, name, cfg_kwargs, batch, pad_fraction, patch_dropout, grad_sample=0):
+    """`grad_sample` > 0: also record each gradient at that many positions (all of a smaller one), drawn
+    without replacement from a generator seeded by the case and parameter names."""
     cfg = O.ClipConfig(**cfg_kwargs)
     state = O.protocol_state_dict(cfg, WEIGHT_SEED)
     text, image = O.protocol_inputs(cfg, batch, INPUT_SEED, pad_fraction)
@@ -152,7 +157,66 @@ def run_case(x_clip, name, cfg_kwargs, batch, pad_fraction, patch_dropout):
     if not cfg.use_all_token_embeds:
         out["text_latents"] = lat[0].tolist()
         out["image_latents"] = lat[1].tolist()
+    if grad_sample:
+        out["grad_samples"] = {}
+        for k, g in grads.items():
+            gen = torch.Generator().manual_seed(zlib.crc32(f"{name}/{k}".encode()))
+            idx = torch.randperm(g.numel(), generator=gen)[:grad_sample].sort().values
+            out["grad_samples"][k] = dict(idx=idx.tolist(), val=[float(f"{v:.7g}") for v in g.flatten()[idx].tolist()])
     return out
+
+
+RANDOM_SEEDS = range(16)
+
+
+def draw_random_case(rng: random.Random):
+    """A small random configuration: widths, head counts, depths, sequence lengths, batch sizes, pad
+    fractions, patch dropout and every combination of the loss flags."""
+    heads_t, heads_i = rng.choice([1, 2, 4]), rng.choice([1, 2, 4])
+    patch = rng.choice([8, 16])
+    side = patch * rng.choice([2, 3, 4])
+    cfg = dict(dim_text=64 * rng.choice([1, 2, 4]), dim_image=64 * rng.choice([1, 2, 4]),
+               dim_latent=64 * rng.choice([1, 2, 4]), num_text_tokens=rng.choice([32, 97, 300]),
+               text_enc_depth=rng.choice([1, 2, 3]), text_seq_len=rng.choice([5, 16, 33]), text_heads=heads_t,
+               visual_enc_depth=rng.choice([1, 2]), visual_heads=heads_i, visual_image_size=side,
+               visual_patch_size=patch)
+    flags = dict(decoupled_contrastive_learning=rng.random() < 0.4, extra_latent_projection=rng.random() < 0.4,
+                 use_all_token_embeds=rng.random() < 0.3)
+    # (FILIP with a causal text tower does not run in the reference itself: 15 text tokens after the CLS
+    #  strip against a 16-wide mask, x_clip.py:705 / :806)
+    text_kind = rng.choice(["plain", "plain", "rotary"] + ([] if flags["use_all_token_embeds"] else ["causal"]))
+    if text_kind == "rotary":
+        flags["text_rotary_pos_emb"] = True
+    elif text_kind == "causal":
+        flags.update(text_causal_mask=True, text_eos_id=cfg["num_text_tokens"] - 1)
+    cfg.update({k: v for k, v in flags.items() if v})
+    batch = rng.choice([2, 3, 5, 8])
+    pad = rng.choice([0.0, 0.2, 0.5])
+    n_patches = (side // patch) ** 2
+    drop = rng.choice([0.0, 0.0, 0.5]) if n_patches >= 4 else 0.0
+    return cfg, batch, pad, drop
+
+
+def random_cases(x_clip):
+    """The reference on the configurations draw_random_case() gives for RANDOM_SEEDS (rng seed 1000 + seed)."""
+    torch.set_num_threads(4)
+    out = []
+    for seed in RANDOM_SEEDS:
+        cfg_kwargs, batch, pad, drop = draw_random_case(random.Random(1000 + seed))
+        r = run_case(x_clip, f"random_{seed}", cfg_kwargs, batch, pad, drop, grad_sample=16)
+        out.append({k: r[k] for k in ("case", "cfg", "batch", "pad_fraction", "patch_dropout", "weight_seed",
+                                      "input_seed", "loss", "dtemperature", "grad_norm", "grad_norms", "grad_samples",
+                                      "enc_text", "enc_image", "latents", "keep")})
+    return out
+
+
+def reference_signature(x_clip):
+    """Keyword names and defaults of the reference's CLIP.__init__ / CLIP.forward, in order; a
+    parameter without a default has no "default" entry."""
+    def params(fn):
+        return [{"name": k} if v.default is inspect.Parameter.empty else {"name": k, "default": v.default}
+                for k, v in inspect.signature(fn).parameters.items() if k not in ("self", "kwargs")]
+    return {"init": params(x_clip.CLIP.__init__), "forward": params(x_clip.CLIP.forward)}
 
 
 def multiview_case(x_clip, name, cfg_kwargs, batch, n_aug_text, n_aug_image):
@@ -286,6 +350,8 @@ def main():
         out = sharded_case(name, cfgk)
         (HERE / f"{name}.json").write_text(json.dumps(out))
         print(name, [(r["loss"], r["grad_norm"], r["dtemperature"]) for r in out["ranks"]])
+    (HERE / "random_cases.json").write_text(json.dumps(random_cases(x_clip), separators=(",", ":")))
+    (HERE / "reference_signature.json").write_text(json.dumps(reference_signature(x_clip), indent=1))
 
 
 if __name__ == "__main__":

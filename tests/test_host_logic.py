@@ -95,26 +95,22 @@ def test_patch_dropout_matches_reference_recipe():
 
 def test_constructor_and_forward_signatures_match_the_reference():
     """Drop-in surface (SURVEY 8b): same keyword names and defaults as x_clip.CLIP.__init__ /
-    forward (x_clip/x_clip.py:413-456, 597-609).  Needs the reference checkout (build container
-    only); skipped where /root/reference is absent (GPU box)."""
-    import importlib
+    forward (x_clip/x_clip.py:413-456, 597-609), as recorded from the reference in
+    tests/golden/reference_signature.json."""
     import inspect
-    import os
-    import sys
-    if not os.path.isdir("/root/reference/x_clip"):
-        pytest.skip("reference checkout not present")
-    sys.path.insert(0, "/root/reference")
-    try:
-        ref = importlib.import_module("x_clip")
-    finally:
-        sys.path.remove("/root/reference")
+    import json
+    from pathlib import Path
     import x_clip_b200
 
     def params(fn):
         return {k: v.default for k, v in inspect.signature(fn).parameters.items()
                 if k not in ("self", "kwargs")}
 
-    ref_init, our_init = params(ref.CLIP.__init__), params(x_clip_b200.CLIP.__init__)
+    def recorded(entries):
+        return {e["name"]: e.get("default", inspect.Parameter.empty) for e in entries}
+
+    sig = json.loads((Path(__file__).parent / "golden" / "reference_signature.json").read_text())
+    ref_init, our_init = recorded(sig["init"]), params(x_clip_b200.CLIP.__init__)
     missing = [k for k in ref_init if k not in our_init]
     assert not missing, f"constructor keywords of the reference missing here: {missing}"
     for k, v in ref_init.items():
@@ -124,6 +120,6 @@ def test_constructor_and_forward_signatures_match_the_reference():
             assert our_init[k] == v, f"default of {k}: reference {v!r}, here {our_init[k]!r}"
     extra = sorted(set(our_init) - set(ref_init))
     assert extra == ["microbatch", "microbatch_retain"], f"unexpected extra constructor keywords: {extra}"
-    ref_fwd, our_fwd = params(ref.CLIP.forward), params(x_clip_b200.CLIP.forward)
+    ref_fwd, our_fwd = recorded(sig["forward"]), params(x_clip_b200.CLIP.forward)
     assert list(ref_fwd) == list(our_fwd), (list(ref_fwd), list(our_fwd))
     assert ref_fwd == our_fwd
