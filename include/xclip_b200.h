@@ -45,17 +45,8 @@ int xclip_init(void);
 /* number of kernels this library has launched since the last reset (host counter) */
 long long xclip_launch_count(void);
 void xclip_launch_count_reset(void);
-/* Explicit, process-wide tuning switches for A/B measurements (never read from the environment;
- * results are identical either way).  Returns the previous value, -1 for an unknown knob.
- *   XCLIP_TUNE_FF_BWD_VARIANT (0): xclip_ff_bwd epilogue: 0 = u by ld.global -> st.shared per step,
- *                                  1 (default) = u by TMA one and a half steps ahead into one of three
- *                                  rotating box sets (0.346 -> 0.297 ms at [50176 x 768], bit-identical)
- *   XCLIP_TUNE_ATTN_SMALL_CTAS (1): resident CTAs per SM of the n <= 128 attention forward, 0 = built-in */
-#define XCLIP_TUNE_FF_BWD_VARIANT 0
-#define XCLIP_TUNE_ATTN_SMALL_CTAS 1
-#define XCLIP_TUNE_ATTN_SMALL_PREFETCH 2 /* n <= 128 attention: next item towards L2 by TMA prefetch (default 0) */
-#define XCLIP_TUNE_LN_FWD_BLOCKS 3 /* LayerNorm forward: cap on resident blocks per SM (0 = built-in 8) */
-#define XCLIP_TUNE_LN_BWD_BLOCKS 4 /* LayerNorm backward: blocks per SM (0 = built-in 2) */
+/* Tuning switches: returns the previous value, -1 for an unknown knob.  No knobs are left, so every
+ * call returns -1 and changes nothing (kept for callers of ABI version 1, e.g. bench.py --tune). */
 int xclip_tune_set(int knob, int value);
 
 /* ---- dense contraction (tcgen05) --------------------------------------
@@ -97,13 +88,6 @@ int xclip_layernorm_bwd(const void* dy, int64_t lddy, const void* x, int64_t ldx
                         const float* stats, const float* g, const void* add, int64_t ldadd,
                         void* dx, int64_t lddx, float* dg, int rows, int d,
                         xclip_stream_t stream);
-/* GEGLU + LayerNorm of FeedForward (x_clip/x_clip.py:180-183,:193): u = [value | gate] bf16
- * [rows, 2*dh]; h = LN(value * gelu_erf(gate)) * g, bf16 [rows, dh]; dh in 1024*{1,2,3,4}. */
-int xclip_geglu_ln_fwd(const void* u, int64_t ldu, const float* g, void* h, int64_t ldh,
-                       float* stats, int rows, int dh, float eps, xclip_stream_t stream);
-int xclip_geglu_ln_bwd(const void* dh_grad, int64_t lddh, const void* u, int64_t ldu,
-                       const float* stats, const float* g, void* du, int64_t lddu, float* dg,
-                       int rows, int dh, xclip_stream_t stream);
 /* l2norm = F.normalize(dim=-1, eps=1e-12) (x_clip/x_clip.py:54-55, used at :715,:724).
  * p f32 [rows,d] -> z f32 [rows,d], inv = 1/max(|p|,eps), and the split-bf16 operands of the
  * logits contraction: zrow = [hi|lo|hi], zcol = [hi|hi|lo], bf16 [rows,3d], hi = bf16(z),

@@ -27,10 +27,10 @@ def test_header_symbols_exported_and_bound():
         assert n in names, f"{n} bound in python but not declared in the header"
 
 
-def test_version_and_error_string_without_gpu():
+def test_abi_version_and_error_string_without_gpu():
     from x_clip_b200 import _lib
     lib = _lib.load()
-    assert lib.xclip_abi_version() == 1
+    assert lib.xclip_abi_version() == 2
     assert isinstance(lib.xclip_last_error(), bytes)
     assert lib.xclip_nce_num_col_blocks(1024) == 4
     assert lib.xclip_nce_num_col_blocks(100) == 1

@@ -53,18 +53,7 @@ def test_ff_forward_and_w2_gradient(cuda_device, M, d):
     (_ln(hp_a, g4_leaf) @ w2_leaf.t()).backward(dx.float())
 
     dxs, vsum, ab = K.ff_bwd_prep(dx, stats, acc, colvec)
-    # both epilogue variants of the fused backward (explicit A/B switch, include/xclip_b200.h): same numbers
-    from x_clip_b200 import _lib
-    lib = _lib.load()
-    prev = lib.xclip_tune_set(0, 0)
-    try:
-        du0 = K.ff_bwd(dx, w2g, u, stats, ab)
-        lib.xclip_tune_set(0, 1)
-        du = K.ff_bwd(dx, w2g, u, stats, ab)
-    finally:
-        lib.xclip_tune_set(0, prev)
-    torch.cuda.synchronize()
-    assert torch.equal(du0, du), "ff_bwd: the TMA-pipelined epilogue must reproduce the ld.global one bit for bit"
+    du = K.ff_bwd(dx, w2g, u, stats, ab)
     raw = torch.zeros(d, 4 * d, device=dev)
     K.gemm(dxs, hp, a_major=1, b_major=1, out=raw, accumulate=True)
     dg4 = torch.zeros(4 * d, device=dev)

@@ -1,14 +1,14 @@
 #!/usr/bin/env python
 """Interleaved A/B timing of whole benchmark steps in ONE process on ONE model (cfg3 by default).
 
-    python tools/ab_step.py "mb=512,retain=auto" "mb=768,retain=auto" "mb=512,retain=auto,tune=0:0" ...
+    python tools/ab_step.py "mb=512,retain=auto" "mb=768,retain=auto" "mb=512,retain=auto,accum=0" ...
 
 Boxes differ by several percent in sustained clocks under the power cap, and one box drifts while it
 warms up, so configurations are compared round-robin (A B C A B C ...) inside one process: `rounds`
 passes over the list, each entry 1 untimed + `steps` timed steps, CUDA events.  Keys: mb (micro-batch),
-retain ("auto" | int), tune ("knob:value;knob:value" -> xclip_tune_set), accum (0/1: in-place gradient
-accumulation of the non-final chunks), alloc ("expandable": torch allocator expandable segments - must be
-the same for every entry, applied at start).  Diagnostic tool - never a bench value."""
+retain ("auto" | int), accum (0/1: in-place gradient accumulation of the non-final chunks), alloc
+("expandable": torch allocator expandable segments - must be the same for every entry, applied at start).
+Diagnostic tool - never a bench value."""
 from __future__ import annotations
 
 import json
@@ -21,7 +21,7 @@ sys.path.insert(0, str(ROOT))
 
 
 def parse(spec):
-    d = dict(mb=512, retain="auto", tune="", accum=1)
+    d = dict(mb=512, retain="auto", accum=1)
     for kv in filter(None, spec.split(",")):
         k, v = kv.split("=")
         d[k] = v
@@ -41,26 +41,18 @@ def main():
         os.environ["PYTORCH_CUDA_ALLOC_CONF"] = "expandable_segments:True"
     import torch
     import bench
-    from x_clip_b200 import _lib, engine
+    from x_clip_b200 import engine
     cfgs = [parse(a) for a in args] or [parse("")]
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(0)
-    lib = _lib.load()
     run = bench.Runner(bench.WORKLOADS[workload][0], "nce", batch, cfgs[0]["mb"], 0.5, dev, 0, 1,
                        retain=cfgs[0]["retain"])
-    defaults = {}
     results = [[] for _ in cfgs]
     for r in range(rounds):
         for i, c in enumerate(cfgs):
             run.clip.microbatch = c["mb"]
             run.clip.microbatch_retain = c["retain"]
             engine.INPLACE_GRAD_ACCUMULATION = bool(c["accum"])
-            for k, v in defaults.items():
-                lib.xclip_tune_set(k, v)
-            for kv in filter(None, c["tune"].split(";")):
-                k, v = kv.split(":")
-                prev = lib.xclip_tune_set(int(k), int(v))
-                defaults.setdefault(int(k), prev)
             run.step()
             torch.cuda.synchronize()
             s0 = torch.cuda.memory_stats(dev)

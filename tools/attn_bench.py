@@ -9,13 +9,7 @@ import sys
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from x_clip_b200 import _lib, kernels as K  # noqa: E402
-
-# tool-side A/B switches: XCLIP_TOOLS_TUNE="knob=value,knob=value" -> xclip_tune_set (the LIBRARY reads
-# no environment variables; this is the measuring script choosing a variant)
-for kv in filter(None, os.environ.get("XCLIP_TOOLS_TUNE", "").split(",")):
-    k, v = kv.split("=")
-    _lib.load().xclip_tune_set(int(k), int(v))
+from x_clip_b200 import kernels as K  # noqa: E402
 
 dev = torch.device("cuda:0")
 shapes = [(512, 98, 12), (512, 78, 8), (1024, 32, 8), (1024, 257, 8), (512, 196, 12)]

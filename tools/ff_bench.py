@@ -1,4 +1,4 @@
-"""Time the pieces of the feed-forward block: fused (csrc/ff.cu) vs separate kernels.
+"""Time the pieces of the fused feed-forward block (csrc/ff.cu) and the GEMMs of its backward.
 
     python tools/ff_bench.py [M,d ...]     (default: cfg3 ViT micro-batch 512, cfg3 text, cfg2 text)"""
 import os
@@ -7,13 +7,7 @@ import sys
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from x_clip_b200 import _lib, kernels as K  # noqa: E402
-
-# tool-side A/B switches: XCLIP_TOOLS_TUNE="knob=value,knob=value" -> xclip_tune_set (the LIBRARY reads
-# no environment variables; this is the measuring script choosing a variant)
-for kv in filter(None, os.environ.get("XCLIP_TOOLS_TUNE", "").split(",")):
-    k, v = kv.split("=")
-    _lib.load().xclip_tune_set(int(k), int(v))
+from x_clip_b200 import kernels as K  # noqa: E402
 
 dev = torch.device("cuda:0")
 shapes = [(512 * 98, 768), (512 * 78, 512), (263168, 512)]
@@ -41,24 +35,16 @@ for (M, d) in shapes:
     g4 = torch.ones(4 * d, device=dev)
     res = torch.randn(M, d, generator=g).to(dev).bfloat16()
     dx = torch.randn(M, d, generator=g).to(dev).bfloat16()
-    w1b, w2b = w1.bfloat16(), w2.bfloat16()
+    w1b = w1.bfloat16()
     w1p, w2g, colvec = K.ff_weights(w1, w2, g4)
     u, hp, rowsum = K.ff_up(x, w1p)
     x2, acc, stats = K.ff_down(hp, w2g, colvec, rowsum, res, 1e-5)
-    h, st = K.geglu_ln_fwd(u, g4)
-    dh = K.gemm(dx, w2b, b_major=1)
     t = {}
-    t["gemm up (plain)"] = timeit(lambda: K.gemm(x, w1b))
     t["ff_up (fused GEGLU)"] = timeit(lambda: K.ff_up(x, w1p))
-    t["geglu_ln_fwd"] = timeit(lambda: K.geglu_ln_fwd(u, g4))
-    t["gemm down (plain)"] = timeit(lambda: K.gemm(h, w2b, residual=res))
     t["ff_down (fused LN)"] = timeit(lambda: K.ff_down(hp, w2g, colvec, rowsum, res, 1e-5))
-    t["gemm dgrad down (plain)"] = timeit(lambda: K.gemm(dx, w2b, b_major=1))
-    t["geglu_ln_bwd"] = timeit(lambda: K.geglu_ln_bwd(dh, u, st, g4))
     t["ff_bwd_prep"] = timeit(lambda: K.ff_bwd_prep(dx, stats))
     t["gemm wgrad up (plain, split-K fp32)"] = timeit(lambda: K.gemm(u, x, a_major=1, b_major=1, accumulate=True))
     t["gemm dgrad up (plain)"] = timeit(lambda: K.gemm(u, w1b, b_major=1))
-    if hasattr(K, "ff_bwd"):
-        dxs, vsum, ab = K.ff_bwd_prep(dx, stats, acc, colvec)
-        t["ff_bwd (fused dgrad + LN/GEGLU bwd)"] = timeit(lambda: K.ff_bwd(dx, w2g, u, stats, ab))
+    dxs, vsum, ab = K.ff_bwd_prep(dx, stats, acc, colvec)
+    t["ff_bwd (fused dgrad + LN/GEGLU bwd)"] = timeit(lambda: K.ff_bwd(dx, w2g, u, stats, ab))
     print(f"M={M} d={d}: " + " | ".join(f"{k} {v:.3f} ms" for k, v in t.items()), flush=True)

@@ -44,10 +44,6 @@ SIGNATURES = {
     "xclip_layernorm_bwd": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
                                     c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int, c_int,
                                     c_void_p]),
-    "xclip_geglu_ln_fwd": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
-                                   c_int, c_int, c_float, c_void_p]),
-    "xclip_geglu_ln_bwd": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
-                                   c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p]),
     "xclip_l2norm_fwd": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                  c_int, c_void_p]),
     "xclip_l2norm_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),

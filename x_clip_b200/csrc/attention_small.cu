@@ -34,7 +34,6 @@ struct AttnSmallFwdParams {
   bf16* o;
   long long ldo;
   float* lse;              // [B, H, n] base-2 log-sum-exp of the scaled, masked scores
-  int prefetch;            // A/B: pull the CTA's next item towards L2 while this one is computed
 };
 
 __device__ __forceinline__ float sm_ex2(float x) {
@@ -177,15 +176,6 @@ attn_fwd_small_kernel(const __grid_constant__ CUtensorMap tm_qkv, const AttnSmal
         tma_load_3d(sK, &tm_qkv, qk_bar, inner + h * kSDh, 0, b);
         mbar_arrive_expect_tx(v_bar, kBox);
         tma_load_3d(sV, &tm_qkv, v_bar, 2 * inner + h * kSDh, 0, b);
-        if (p.prefetch) {   // the CTA's NEXT item travels HBM -> L2 while this one is computed
-          const int bh2 = bh + (int)gridDim.x;
-          if (bh2 < total) {
-            const int b2 = bh2 / p.H, h2 = bh2 - b2 * p.H;
-            tma_prefetch_l2_3d(&tm_qkv, h2 * kSDh, 0, b2);
-            tma_prefetch_l2_3d(&tm_qkv, inner + h2 * kSDh, 0, b2);
-            tma_prefetch_l2_3d(&tm_qkv, 2 * inner + h2 * kSDh, 0, b2);
-          }
-        }
         if (it > 0) mbar_wait(e_bar, par ^ 1);   // O of the previous item was read out of TMEM
         mbar_wait(qk_bar, par);
         tcgen05_fence_after();
@@ -407,9 +397,7 @@ static int launch_fwd_small(const void* qkv, int64_t ld_qkv, const AttnSmallFwdP
   auto kern = attn_fwd_small_kernel<ROWS, kCausal>;
   rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), kSmem);
   if (rc) return rc;
-  int per_sm = tune(XCLIP_TUNE_ATTN_SMALL_CTAS);          // A/B switch: fewer co-resident CTAs
-  if (per_sm <= 0 || per_sm > kPerSm) per_sm = kPerSm;
-  long long grid = (long long)num_sms() * per_sm;
+  long long grid = (long long)num_sms() * kPerSm;
   if (grid > (long long)p.B * p.H) grid = (long long)p.B * p.H;
   kern<<<(int)grid, kThreads, kSmem, stream>>>(tm, p);
   XCLIP_LAUNCH_CHECK("attn_fwd_small_kernel");
@@ -427,7 +415,6 @@ struct AttnSmallBwdParams {
   const float* delta;    // [B, H, n] rowsum(dO * O)
   bf16* dqkv;            // [B*n, ld]: dq | dk | dv
   long long ld;
-  int prefetch;          // A/B: next item towards L2 (see the forward kernel)
 };
 
 constexpr int kSBwdComputeWarps = 8;
@@ -527,16 +514,6 @@ attn_bwd_small_kernel(const __grid_constant__ CUtensorMap tm_qkv,
         mbar_arrive_expect_tx(vdo_bar, 2 * box);
         tma_load_3d(sP, &tm_qkv, vdo_bar, 2 * inner + h * kSDh, 0, b);
         tma_load_3d(sdO, &tm_do, vdo_bar, h * kSDh, 0, b);
-        if (p.prefetch) {
-          const int bh2 = bh + (int)gridDim.x;
-          if (bh2 < total) {
-            const int b2 = bh2 / p.H, h2 = bh2 - b2 * p.H;
-            tma_prefetch_l2_3d(&tm_qkv, h2 * kSDh, 0, b2);
-            tma_prefetch_l2_3d(&tm_qkv, inner + h2 * kSDh, 0, b2);
-            tma_prefetch_l2_3d(&tm_qkv, 2 * inner + h2 * kSDh, 0, b2);
-            tma_prefetch_l2_3d(&tm_do, h2 * kSDh, 0, b2);
-          }
-        }
         if (it > 0) mbar_wait(e_bar, par ^ 1);   // dQ/dK/dV of the previous item left TMEM
         mbar_wait(qk_bar, par);
         tcgen05_fence_after();
@@ -743,7 +720,6 @@ int attn_bwd_small(const void* qkv, int64_t ld_qkv, const uint8_t* key_mask, con
   p.scale = scale; p.scale_log2 = scale * 1.4426950408889634f;
   p.mask = key_mask; p.lse = lse; p.delta = delta;
   p.dqkv = reinterpret_cast<bf16*>(dqkv); p.ld = ld_dqkv;
-  p.prefetch = tune(XCLIP_TUNE_ATTN_SMALL_PREFETCH);
   CUtensorMap tq, tdo;
   int rc = encode_3d_bf16(&tq, qkv, (uint64_t)(3 * heads * kSDh), (uint64_t)n, (uint64_t)B,
                           (uint64_t)ld_qkv, (uint64_t)n * ld_qkv, kSDh, (uint32_t)p.nkp);
@@ -782,7 +758,6 @@ int attn_fwd_small(const void* qkv, int64_t ld_qkv, const uint8_t* key_mask, voi
   p.o = reinterpret_cast<bf16*>(o);
   p.ldo = ldo;
   p.lse = lse;
-  p.prefetch = tune(XCLIP_TUNE_ATTN_SMALL_PREFETCH);
   if (n <= 64)
     return causal ? launch_fwd_small<64, true>(qkv, ld_qkv, p, stream)
                   : launch_fwd_small<64, false>(qkv, ld_qkv, p, stream);

@@ -143,15 +143,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-// pull a tensor box towards L2 (no shared memory, no barrier): the later tma_load of the same box
-// then sees L2 instead of HBM latency
-__device__ __forceinline__ void tma_prefetch_l2_3d(const CUtensorMap* m, int32_t c0, int32_t c1, int32_t c2) {
-  asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global [%0, {%1, %2, %3}];" ::"l"(
-                   reinterpret_cast<uint64_t>(m)),
-               "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
-
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m, uint64_t* bar,
                                             int32_t c0, int32_t c1, int32_t c2) {
   asm volatile(
@@ -339,38 +330,6 @@ __device__ __forceinline__ uint32_t swz128(uint32_t row, uint32_t c16) {
 }
 
 // ---------------------------------------------------------------------------
-// GELU (erf form, x_clip/x_clip.py:183 F.gelu) shared by the row-wise kernels and the fused
-// feed-forward GEMM epilogues
-// ---------------------------------------------------------------------------
-// erf by Abramowitz & Stegun 7.1.26 (|error| <= 1.5e-7, far below bf16 output resolution):
-// one MUFU.RCP + one MUFU.EX2 + 6 FMA instead of libdevice erff's ~25 instructions.  The GEGLU
-// kernels would otherwise be instruction-bound, not HBM-bound.  exp(-x^2/2) is shared with the
-// Gaussian density that gelu'(x) needs.
-struct GeluParts {
-  float cdf;   // Phi(x) = 0.5 * (1 + erf(x / sqrt(2)))
-  float pdf;   // phi(x) = exp(-x^2/2) / sqrt(2 pi)
-};
-__device__ __forceinline__ GeluParts gelu_parts(float x) {
-  const float z = fabsf(x) * 0.70710678118654752f;            // |x| / sqrt(2)
-  float t;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(fmaf(0.3275911f, z, 1.f)));
-  float poly = fmaf(1.061405429f, t, -1.453152027f);
-  poly = fmaf(poly, t, 1.421413741f);
-  poly = fmaf(poly, t, -0.284496736f);
-  poly = fmaf(poly, t, 0.254829592f);
-  poly *= t;
-  float e_half;                                                // exp(-x^2/2) == exp(-z^2)
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e_half) : "f"(-0.72134752044448170f * x * x));
-  const float erfc_z = poly * e_half;
-  const float half_erfc = 0.5f * erfc_z;
-  GeluParts g;
-  g.cdf = x >= 0.f ? 1.f - half_erfc : half_erfc;
-  g.pdf = 0.3989422804014327f * e_half;
-  return g;
-}
-__device__ __forceinline__ float gelu_erf(float x) { return x * gelu_parts(x).cdf; }
-
-// ---------------------------------------------------------------------------
 // Packed fp32x2 arithmetic (sm_100: FFMA2 - one instruction, one issue slot, two IEEE fp32 FMAs on
 // an aligned register pair).  The GELU epilogues of the fused feed-forward are bound by the FMA pipe
 // (~28 FMA-class instructions per element in scalar form against 2 MUFU); in packed form the
@@ -411,7 +370,13 @@ __device__ __forceinline__ uint32_t f2_to_bf16x2(f32x2 v) {
   return pack_bf16x2(lo, hi);
 }
 
-// gelu_parts for two elements at once: cdf = Phi(x), pdf = phi(x) (same A&S 7.1.26 polynomial).
+// ---------------------------------------------------------------------------
+// GELU (erf form, x_clip/x_clip.py:183 F.gelu) for the fused feed-forward GEMM epilogues, two elements
+// at once: cdf = Phi(x) = 0.5 * (1 + erf(x / sqrt(2))), pdf = phi(x) = exp(-x^2/2) / sqrt(2 pi).
+// erf by Abramowitz & Stegun 7.1.26 (|error| <= 1.5e-7, far below bf16 output resolution): one
+// MUFU.RCP + one MUFU.EX2 + 6 FMA per element instead of libdevice erff's ~25 instructions.
+// exp(-x^2/2) is shared with the Gaussian density that gelu'(x) needs.
+// ---------------------------------------------------------------------------
 struct GeluParts2 {
   f32x2 cdf, pdf;
 };

@@ -3,7 +3,7 @@
 //   x2 = LN_4d(hp) g W2^T + x1                     one GEMM, LayerNorm folded into
 //                                                  weight + epilogue                (xclip_ff_down)
 // so the [tokens, 8d] / [tokens, 4d] hidden activations make no extra round trip through HBM for
-// the activation and the normalisation (the separate geglu_ln_fwd kernel was 10 % of the cfg3 step
+// the activation and the normalisation (a separate GEGLU + LayerNorm pass was 10 % of the cfg3 step
 // and instruction-issue bound).  The LayerNorm fold:
 //   LN(hp)_k g_k = (hp_k - mean) rstd g_k   =>   x2_j = rstd (sum_k hp_k W2g_jk - mean c_j),
 //   W2g = W2 . g (column scaling), c_j = sum_k W2g_jk.
@@ -181,9 +181,6 @@ extern "C" int xclip_ff_bwd(const void* dx, int64_t lddx, const void* w2g, const
   GemmParams p = {};
   p.M = M; p.N = 4 * d; p.K = d; p.split_k = 1; p.alpha = 1.f;
   p.ff_stats = const_cast<float*>(stats); p.ff_ab = ab; p.ff_hidden = 4 * d;
-  p.ff_u = reinterpret_cast<const bf16*>(u); p.ff_ldu = ldu;
-  if (tune(XCLIP_TUNE_FF_BWD_VARIANT) == 0)      // older epilogue: u by ld.global -> st.shared (kept for A/B)
-    return launch_pair_ff<PEPI_FF_BWD, kMajorMN>(tmA, tmB, tmC, tmC, p, reinterpret_cast<cudaStream_t>(stream));
   CUtensorMap tmU;                               // u = [value | gate], loaded box-wise ahead of its step
   if ((rc = encode_2d_bf16(&tmU, u, (uint64_t)(8 * d), (uint64_t)M, (uint64_t)ldu, 64, kGemmBlockM))) return rc;
   return launch_pair_ff<PEPI_FF_BWD2, kMajorMN>(tmA, tmB, tmC, tmU, p, reinterpret_cast<cudaStream_t>(stream));

@@ -65,8 +65,6 @@ struct GemmParams {
   float ff_eps;            // LayerNorm epsilon
   int ff_hidden;           // 4*dim: LayerNorm width; column offset of the gate half inside u
   int ff_skip_u;           // UP: do not write u = [value | gate] (inference / no-grad sweeps need only hp)
-  const bf16* ff_u;        // BWD: saved [value | gate] activations [M, 8d]
-  long long ff_ldu;
   const float* ff_ab;      // BWD: [M,2] per-row (mean_k(gdh), mean_k(gdh * hn)) from xclip_ff_bwd_prep
 };
 

@@ -23,14 +23,14 @@
 //                x2 = LN(hp) g W2^T + x1 = rstd_r (acc_rj - mean_r c_j) + x1_rj  with
 //                acc = hp (W2 . g)^T and c_j = sum_k (W2 . g)_jk; also writes bf16(acc) and
 //                (mean, rstd) for the backward.
-//   PEPI_FF_BWD  backward of LayerNorm(4d) + GEGLU fused into the down-projection's dgrad GEMM
+//   PEPI_FF_BWD2 backward of LayerNorm(4d) + GEGLU fused into the down-projection's dgrad GEMM
 //                gdh = dx (W2 . g): per element
 //                  hn = (value*gelu(gate) - mean) rstd;  dhp = rstd (gdh - a_r - hn b_r)
 //                  d value = dhp gelu(gate);  d gate = dhp value gelu'(gate)
 //                with the two row means a_r = mean_k gdh, b_r = mean_k gdh*hn supplied by
 //                xclip_ff_bwd_prep (they only need the d-wide vectors dx, W2g row sums and the saved
-//                down-projection accumulator).  Reads u = [value | gate], writes du - the [M, 4d]
-//                gradient dh and the separate geglu_ln_bwd pass disappear.
+//                down-projection accumulator).  Reads u = [value | gate] by TMA one and a half steps
+//                ahead, writes du - the [M, 4d] gradient dh never exists.
 #pragma once
 
 #include "gemm.cuh"
@@ -40,15 +40,14 @@ namespace xclip {
 constexpr int PEPI_STORE = 0;
 constexpr int PEPI_FF_UP = 1;
 constexpr int PEPI_FF_DOWN = 2;
-constexpr int PEPI_FF_BWD = 3;
-constexpr int PEPI_FF_BWD2 = 4;   // same math as PEPI_FF_BWD, u arrives by TMA one step ahead (see the epilogue)
+constexpr int PEPI_FF_BWD2 = 4;
 
 template <int EPI>
 struct PairCfg {
   // the GELU epilogues are latency-bound (two MUFU + a dependent polynomial per element): with two
   // warps per scheduler ncu showed 36 % issue-slot and 33 % XU utilisation while the tensor pipe idled
   // a third of the time, so they get four warps per scheduler
-  static constexpr int kEpiWarps = (EPI == PEPI_FF_UP || EPI == PEPI_FF_BWD || EPI == PEPI_FF_BWD2) ? 16 : 4;
+  static constexpr int kEpiWarps = (EPI == PEPI_FF_UP || EPI == PEPI_FF_BWD2) ? 16 : 4;
   static constexpr int kThreads = (kEpiWarps + 2) * 32;
   static constexpr int kABytes = kGemmBlockM * kGemmBlockK * 2;   // 16 KiB: this CTA's 128 rows of A
   static constexpr int kBBytes = 128 * kGemmBlockK * 2;           // 16 KiB: this CTA's 128 of 256 N columns
@@ -57,10 +56,10 @@ struct PairCfg {
   // STORE: 2 boxes (double buffered); FF_UP: one box per column half (value, gate and hp pass through it
   // one after the other - they wait in registers; a second box per half was measured: it removes the
   // barrier stalls but costs the sixth mainloop stage, 0.366 -> 0.384 ms at K = 768); FF_DOWN: two
-  // (out, acc) box pairs alternating by 64-column step; FF_BWD: (d value, d gate) x 2 halves
-  // FF_BWD2: three SETS of (value, gate) boxes rotate through "being loaded by TMA / worked on / being
-  // stored" - paid for with one mainloop stage (with three stages the epilogue waited for the MMAs,
-  // with four it does not: the dgrad GEMM has K = d <= 1024 and the kernel is bound by its epilogue)
+  // (out, acc) box pairs alternating by 64-column step; FF_BWD2: three SETS of (value, gate) boxes
+  // rotate through "being loaded by TMA / worked on / being stored" - paid for with one mainloop stage
+  // (with three stages the epilogue waited for the MMAs, with four it does not: the dgrad GEMM has
+  // K = d <= 1024 and the kernel is bound by its epilogue)
   static constexpr int kStagingBytes =
       (EPI == PEPI_FF_BWD2 ? 6 : (EPI == PEPI_STORE || EPI == PEPI_FF_UP) ? 2 : 4) * kBox;
   static constexpr int kStages = EPI == PEPI_FF_BWD2 ? 4 : (EPI == PEPI_STORE || EPI == PEPI_FF_UP) ? 6 : 5;
@@ -357,107 +356,16 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           *reinterpret_cast<float2*>(p.ff_rowsum + 2ll * ((long long)row * nparts + n_blk * 2 + bs)) =
               make_float2(s1, s2);
         }
-      } else if constexpr (EPI == PEPI_FF_BWD) {
-        // tile columns = hidden units [256 n_blk, +256).  16 warps: sub = warp>>2; half = sub>>1 owns
-        // columns [128 half, +128) in two 64-column groups; the two subs of a half split each group
-        // (32 columns each).  u = [value | gate] is read COALESCED into the staging boxes, which have
-        // exactly the layout the TMA store wants (rows of a lane quarter are private to the two warps
-        // that share it); each lane then picks up its row and the gradients overwrite it in place.
-        // (A lane reading its own row straight from global memory costs 32 L1 wavefronts per request -
-        // 8 k cycles per tile, more than the tile's MMAs.)
-        const int sub = warp >> 2;
-        const int bhalf = sub >> 1;
-        const int part = sub & 1;                                      // which 32 columns of a group
-        const uint32_t stg = smem_u32(smem_c) + bhalf * 2 * S::kBox;   // value -> d value | gate -> d gate
-        const bool issuer = (threadIdx.x == bhalf * 256);
-        float mean = 0.f, rstd = 0.f, am = 0.f, bm = 0.f;
-        if (row_ok) {
-          const float2 st = *reinterpret_cast<const float2*>(p.ff_stats + 2ll * row);
-          const float2 ab = *reinterpret_cast<const float2*>(p.ff_ab + 2ll * row);
-          mean = st.x; rstd = st.y; am = ab.x; bm = ab.y;
-        }
-        const f32x2 rstd2 = f2_splat(rstd), nmr = f2_splat(-mean * rstd), namr = f2_splat(-am * rstd),
-                    nbmr = f2_splat(-bm * rstd);
-        const int slab_row0 = m_blk * kGemmBlockM + quarter * 32;      // first global row of the slab
-#pragma unroll 1
-        for (int q = 0; q < 2; ++q) {
-          const int kq = n_blk * BLOCK_N + bhalf * 128 + q * 64;
-          // coalesced fetch: iteration t covers slab rows 4t..4t+3 (this warp: t = 4 part .. 4 part + 3),
-          // lane = (row%4)*8 + 16-byte chunk
-          uint4 rawv[4], rawg[4];
-#pragma unroll
-          for (int t4 = 0; t4 < 4; ++t4) {
-            const int rr = slab_row0 + (part * 4 + t4) * 4 + (lane >> 3);
-            const bf16* src = p.ff_u + (long long)(rr < p.M ? rr : 0) * p.ff_ldu + kq + (lane & 7) * 8;
-            rawv[t4] = *reinterpret_cast<const uint4*>(src);
-            rawg[t4] = *reinterpret_cast<const uint4*>(src + p.ff_hidden);
-          }
-          if (issuer) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-          asm volatile("bar.sync %0, 256;" ::"r"(1 + bhalf) : "memory");   // previous stores have read the boxes
-#pragma unroll
-          for (int t4 = 0; t4 < 4; ++t4) {
-            const int r = quarter * 32 + (part * 4 + t4) * 4 + (lane >> 3);
-            const uint32_t off = swz128(r, lane & 7);
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + off), "r"(rawv[t4].x),
-                         "r"(rawv[t4].y), "r"(rawv[t4].z), "r"(rawv[t4].w) : "memory");
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + S::kBox + off), "r"(rawg[t4].x),
-                         "r"(rawg[t4].y), "r"(rawg[t4].z), "r"(rawg[t4].w) : "memory");
-          }
-          asm volatile("bar.sync %0, 256;" ::"r"(1 + bhalf) : "memory");   // both warps of a quarter filled it
-#pragma unroll
-          for (int c16 = 0; c16 < 2; ++c16) {
-            uint32_t v[16];
-            tmem_ld_32x16(taddr + bhalf * 128 + q * 64 + part * 32 + c16 * 16, v);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; i += 8) {
-              const int chunk = part * 4 + c16 * 2 + (i >> 3);
-              const uint32_t off = swz128(row_in_tile, chunk);
-              uint32_t wv[4], wg[4];
-              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
-                           : "=r"(wv[0]), "=r"(wv[1]), "=r"(wv[2]), "=r"(wv[3]) : "r"(stg + off));
-              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
-                           : "=r"(wg[0]), "=r"(wg[1]), "=r"(wg[2]), "=r"(wg[3]) : "r"(stg + S::kBox + off));
-              uint32_t dvw[4], dgw[4];
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {                           // two columns per step (fp32x2)
-                const float g0 = __uint_as_float(wg[k] << 16), g1 = __uint_as_float(wg[k] & 0xffff0000u);
-                const f32x2 gate = f2_pack(g0, g1), val = f2_from_bf16x2(wv[k]);
-                const GeluParts2 gp = gelu_parts2(g0, g1);
-                const f32x2 ge = f2_mul(gate, gp.cdf);                // gelu(gate)
-                const f32x2 gd = f2_fma(gate, gp.pdf, gp.cdf);        // gelu'(gate)
-                const f32x2 hn = f2_fma(f2_mul(val, ge), rstd2, nmr); // (val*ge - mean) rstd
-                f32x2 dhp = f2_fma(f2_pack(__uint_as_float(v[i + 2 * k]), __uint_as_float(v[i + 2 * k + 1])),
-                                   rstd2, namr);                      // rstd (gdh - a)
-                dhp = f2_fma(hn, nbmr, dhp);                          //   - rstd b hn
-                dvw[k] = f2_to_bf16x2(f2_mul(dhp, ge));
-                dgw[k] = f2_to_bf16x2(f2_mul(f2_mul(dhp, val), gd));
-              }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + off), "r"(dvw[0]),
-                           "r"(dvw[1]), "r"(dvw[2]), "r"(dvw[3]) : "memory");
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + S::kBox + off), "r"(dgw[0]),
-                           "r"(dgw[1]), "r"(dgw[2]), "r"(dgw[3]) : "memory");
-            }
-          }
-          fence_proxy_async_smem();
-          asm volatile("bar.sync %0, 256;" ::"r"(1 + bhalf) : "memory");
-          if (issuer) {
-            const int r0 = m_blk * kGemmBlockM;
-            tma_store_2d(&tmC, stg, kq, r0);                        // du[:, k ..]        d value
-            tma_store_2d(&tmC, stg + S::kBox, p.ff_hidden + kq, r0);   // du[:, 4d + k ..]   d gate
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          }
-        }
       } else if constexpr (EPI == PEPI_FF_BWD2) {
-        // Same arithmetic as PEPI_FF_BWD, different data movement.  The older epilogue fetched u with
-        // ld.global -> st.shared at the start of every 64-column step and its warps then sat on the HBM
-        // latency (ncu: 26 % long-scoreboard at the STS + 22 % barrier stalls behind it).  Here all 16
-        // warps work on one 64-column step at a time (a warp: its 32-row lane quarter x 16 columns) and a
-        // step's (value, gate) boxes arrive by TMA in one of THREE box sets, requested one and a half steps
-        // ahead by thread 0 as soon as the set's previous gradient store has been read:
+        // u is not fetched by ld.global -> st.shared at the start of each 64-column step: the warps then
+        // sit on the HBM latency (ncu: 26 % long-scoreboard at the STS + 22 % barrier stalls behind it;
+        // 0.346 vs 0.297 ms at [50176 x 768]).  Instead all 16 warps work on one 64-column step at a
+        // time (a warp: its 32-row lane quarter x 16 columns) and a step's (value, gate) boxes arrive by
+        // TMA in one of THREE box sets, requested one and a half steps ahead by thread 0 as soon as the
+        // set's previous gradient store has been read:
         //   step g uses set g % 3;   L(g) = TMA load of step g;   S(g) = TMA store of step g
         //   prologue: L(0), L(1);    middle of step g: wait S(<= g-1) read, issue L(g+2)
-        // The gradients overwrite u in place and leave by TMA store as before.
+        // The gradients overwrite u in place and leave by TMA store.
         const int cs = warp >> 2;                                      // which 16 columns of the 64-column step
         const bool issuer = threadIdx.x == 0;
         const float mean = nst.x, rstd = nst.y, am = nab.x, bm = nab.y;
@@ -594,7 +502,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       }
     }
     // outstanding TMA stores must have READ their staging smem before the CTA exits
-    if (EPI == PEPI_FF_UP || EPI == PEPI_FF_BWD || EPI == PEPI_FF_BWD2) {
+    if (EPI == PEPI_FF_UP || EPI == PEPI_FF_BWD2) {
       if ((threadIdx.x & 255) == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
     } else if ((EPI != PEPI_STORE || p.use_tma_store) && threadIdx.x == 0) {
       asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");

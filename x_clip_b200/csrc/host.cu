@@ -135,21 +135,11 @@ int encode_3d_bf16(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t m
 
 }  // namespace xclip
 
-namespace xclip {
-static int g_tune[8] = {1, 0, 0, 0, 0, 0, 0, 0};   // XCLIP_TUNE_FF_BWD_VARIANT = 1 (TMA-pipelined)
-int tune(int knob) { return (knob >= 0 && knob < 8) ? g_tune[knob] : 0; }
-}  // namespace xclip
-
 extern "C" {
 
-int xclip_tune_set(int knob, int value) {
-  if (knob < 0 || knob >= 8) return -1;
-  const int prev = xclip::g_tune[knob];
-  xclip::g_tune[knob] = value;
-  return prev;
-}
+int xclip_tune_set(int, int) { return -1; }
 
-int xclip_abi_version(void) { return 1; }
+int xclip_abi_version(void) { return 2; }
 
 const char* xclip_last_error(void) { return xclip::g_err; }
 

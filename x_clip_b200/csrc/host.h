@@ -22,9 +22,6 @@ int num_sms();
 // per device, so a process driving several GPUs must set it on each of them
 int ensure_dynamic_smem(const void* kernel, int bytes);
 
-// explicit tuning switches (xclip_tune_set); index = XCLIP_TUNE_*
-int tune(int knob);
-
 // counts kernel launches made by this library (bench.py reports it as gpu_launches)
 void count_launch(int n = 1);
 

@@ -1,6 +1,5 @@
 // Row-wise HBM-bound kernels of the transformer block and the latent head:
 //   gain-only LayerNorm fwd/bwd   (reference x_clip/x_clip.py:112-121; used at :126,:210,:193,:271-272)
-//   GEGLU + LayerNorm fwd/bwd     (reference :180-183 + :193 inside FeedForward :185-199)
 //   l2-normalise fwd/bwd          (reference :54-55, called at :715,:724)
 //   fp32 -> bf16 cast             (weights are kept fp32 by the module; MMA operands are bf16)
 //
@@ -260,139 +259,6 @@ ln_bwd_kernel(const bf16* __restrict__ dy, long long lddy, const bf16* __restric
 }
 
 // ---------------------------------------------------------------------------
-// GEGLU + LayerNorm.  u = [val | gate] (each DH wide).  v = val * gelu_erf(gate)
-//   fwd: h = LN(v) * g ; stats = (mean, rstd) of v
-//   bwd: dv = LN-bwd(dh);  dval = dv * gelu(gate);  dgate = dv * val * gelu'(gate)
-// ---------------------------------------------------------------------------
-// (gelu_parts / gelu_erf live in common.cuh: the GEMM epilogues of the fused feed-forward share them)
-// The hidden width DH = 4*dim is 1024..4096: one ROW per block of DH/8 threads, each thread
-// owns exactly one 16-byte vector of value, gate and gradient (low register count -> many rows
-// in flight per SM, which is what an HBM-bound kernel needs).
-template <int WARPS>
-__device__ __forceinline__ float2 block_sum2(float a, float b, float* scratch /* [2*WARPS] */) {
-  a = warp_sum(a);
-  b = warp_sum(b);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  __syncthreads();  // scratch reuse across calls
-  if (lane == 0) { scratch[warp] = a; scratch[WARPS + warp] = b; }
-  __syncthreads();
-  float ra = 0.f, rb = 0.f;
-#pragma unroll
-  for (int w = 0; w < WARPS; ++w) { ra += scratch[w]; rb += scratch[WARPS + w]; }
-  return make_float2(ra, rb);
-}
-
-template <int THREADS>  // THREADS = DH / 8
-__global__ void __launch_bounds__(THREADS)
-geglu_ln_fwd_kernel(const bf16* __restrict__ u, long long ldu, const float* __restrict__ g,
-                    bf16* __restrict__ h, long long ldh, float* __restrict__ stats, int rows,
-                    float eps) {
-  constexpr int DH = THREADS * 8;
-  constexpr int WARPS = THREADS / 32;
-  __shared__ float scratch[2 * WARPS];
-  const int col = threadIdx.x * 8;
-  float gg[8];
-  loadf8(g + col, gg);
-  // software pipeline: the next row's vectors are in flight while this row is reduced
-  // (block-level syncs otherwise limit the bytes in flight per SM and the kernel becomes
-  // latency- instead of HBM-bound)
-  uint4 nv = make_uint4(0, 0, 0, 0), ng = nv;
-  if (blockIdx.x < rows) {
-    nv = *reinterpret_cast<const uint4*>(u + (long long)blockIdx.x * ldu + col);
-    ng = *reinterpret_cast<const uint4*>(u + (long long)blockIdx.x * ldu + DH + col);
-  }
-  for (int row = blockIdx.x; row < rows; row += gridDim.x) {
-    float v[8], gt[8];
-    unpack8(nv, v);
-    unpack8(ng, gt);
-    const int nrow = row + gridDim.x;
-    if (nrow < rows) {
-      nv = *reinterpret_cast<const uint4*>(u + (long long)nrow * ldu + col);
-      ng = *reinterpret_cast<const uint4*>(u + (long long)nrow * ldu + DH + col);
-    }
-    float s = 0.f, q = 0.f;
-#pragma unroll
-    for (int e = 0; e < 8; ++e) { v[e] *= gelu_erf(gt[e]); s += v[e]; q += v[e] * v[e]; }
-    // one block reduction for both moments: var = E[v^2] - mean^2 (|mean| << std for GEGLU
-    // outputs, so the fp32 cancellation error is ~1e-7 relative)
-    const float2 mom = block_sum2<WARPS>(s, q, scratch);
-    const float mean = mom.x * (1.f / DH);
-    const float rstd = rsqrtf(fmaxf(mom.y * (1.f / DH) - mean * mean, 0.f) + eps);
-    if (threadIdx.x == 0) {
-      stats[2 * (long long)row] = mean;
-      stats[2 * (long long)row + 1] = rstd;
-    }
-    float o[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) o[e] = (v[e] - mean) * rstd * gg[e];
-    store8(h + row * ldh + col, o);
-  }
-}
-
-template <int THREADS>  // THREADS = DH / 8
-__global__ void __launch_bounds__(THREADS, (768 / THREADS) > 0 ? (768 / THREADS) : 1)
-geglu_ln_bwd_kernel(const bf16* __restrict__ dh, long long lddh, const bf16* __restrict__ u,
-                    long long ldu, const float* __restrict__ stats, const float* __restrict__ g,
-                    bf16* __restrict__ du, long long lddu, float* __restrict__ dg, int rows) {
-  constexpr int DH = THREADS * 8;
-  constexpr int WARPS = THREADS / 32;
-  __shared__ float scratch[2 * WARPS];
-  const int col = threadIdx.x * 8;
-  float gg[8], dgacc[8];
-  loadf8(g + col, gg);
-#pragma unroll
-  for (int e = 0; e < 8; ++e) dgacc[e] = 0.f;
-
-  uint4 nv = make_uint4(0, 0, 0, 0), ng = nv, nd = nv;   // next row's vectors (prefetched)
-  if (blockIdx.x < rows) {
-    nv = *reinterpret_cast<const uint4*>(u + (long long)blockIdx.x * ldu + col);
-    ng = *reinterpret_cast<const uint4*>(u + (long long)blockIdx.x * ldu + DH + col);
-    nd = *reinterpret_cast<const uint4*>(dh + (long long)blockIdx.x * lddh + col);
-  }
-  for (int row = blockIdx.x; row < rows; row += gridDim.x) {
-    const float mean = stats[2 * (long long)row], rstd = stats[2 * (long long)row + 1];
-    float va[8], gt[8], gd[8], ge[8], vh[8];
-    unpack8(nv, va);
-    unpack8(ng, gt);
-    unpack8(nd, gd);
-    const int nrow = row + gridDim.x;
-    if (nrow < rows) {
-      nv = *reinterpret_cast<const uint4*>(u + (long long)nrow * ldu + col);
-      ng = *reinterpret_cast<const uint4*>(u + (long long)nrow * ldu + DH + col);
-      nd = *reinterpret_cast<const uint4*>(dh + (long long)nrow * lddh + col);
-    }
-    float s1 = 0.f, s2 = 0.f;
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const GeluParts gp = gelu_parts(gt[e]);
-      ge[e] = gt[e] * gp.cdf;
-      gt[e] = fmaf(gt[e], gp.pdf, gp.cdf);          // gate now holds gelu'(gate)
-      vh[e] = (va[e] * ge[e] - mean) * rstd;
-      dgacc[e] += gd[e] * vh[e];
-      gd[e] *= gg[e];
-      s1 += gd[e];
-      s2 += gd[e] * vh[e];
-    }
-    const float2 ss = block_sum2<WARPS>(s1, s2, scratch);
-    s1 = ss.x * (1.f / DH);
-    s2 = ss.y * (1.f / DH);
-    float o_val[8], o_gate[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const float dv = rstd * (gd[e] - s1 - vh[e] * s2);
-      o_val[e] = dv * ge[e];
-      o_gate[e] = dv * va[e] * gt[e];
-    }
-    store8(du + row * lddu + col, o_val);
-    store8(du + row * lddu + DH + col, o_gate);
-  }
-  if (dg != nullptr) {
-#pragma unroll
-    for (int e = 0; e < 8; ++e) atomicAdd(dg + col + e, dgacc[e]);
-  }
-}
-
-// ---------------------------------------------------------------------------
 // l2-normalise rows of an fp32 matrix: z = p / max(||p||, 1e-12)
 //   fwd writes z (fp32), the split-bf16 MMA operands zrow = [hi|lo|hi], zcol = [hi|hi|lo]
 //   ([rows, 3d] each; zrow . zcol^T reproduces the fp32 dot product to ~2^-17) and
@@ -608,32 +474,12 @@ static int row_grid(int rows) {
   return blocks < cap ? (blocks > 0 ? blocks : 1) : cap;
 }
 
-static int wide_grid(int rows, int dh) {
-  const int per_sm = 2048 / (dh / 8);      // resident blocks per SM at DH/8 threads each
-  const int cap = num_sms() * per_sm;
-  return rows < cap ? rows : cap;
-}
-
 }  // namespace xclip
 
 using namespace xclip;
 
 #define LAUNCH_NV(KERNEL, NVAL, GRID, STREAM, ...) \
   case NVAL: KERNEL<NVAL><<<GRID, kRowThreads, 0, STREAM>>>(__VA_ARGS__); break;
-
-#define LAUNCH_WIDE(KERNEL, THREADS, GRID, STREAM, ...) \
-  case THREADS: KERNEL<THREADS><<<GRID, THREADS, 0, STREAM>>>(__VA_ARGS__); break;
-
-// feed-forward hidden widths 1024*{1,2,3,4} (= 4*dim for dim 256..1024): DH/8 threads per row
-#define DISPATCH_WIDE(KERNEL, D, GRID, STREAM, ...)                                       \
-  switch ((D) / 8) {                                                                      \
-    LAUNCH_WIDE(KERNEL, 128, GRID, STREAM, __VA_ARGS__)                                   \
-    LAUNCH_WIDE(KERNEL, 256, GRID, STREAM, __VA_ARGS__)                                   \
-    LAUNCH_WIDE(KERNEL, 384, GRID, STREAM, __VA_ARGS__)                                   \
-    LAUNCH_WIDE(KERNEL, 512, GRID, STREAM, __VA_ARGS__)                                   \
-    default:                                                                              \
-      return fail(XCLIP_ERR_INVALID, "hidden width %d unsupported (1024*{1,2,3,4})", (D)); \
-  }
 
 #define DISPATCH_NARROW(KERNEL, D, GRID, STREAM, ...)                                     \
   switch ((D) / 256) {                                                                    \
@@ -662,10 +508,7 @@ extern "C" int xclip_layernorm_fwd(const void* x, int64_t ldx, const float* g, c
                     (!g2 || (ALIGNED16(g2) && out2 && ALIGNED16(out2))),
                 "layernorm_fwd: pointers must be 16-byte aligned");
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  int fgrid = row_grid(rows);
-  if (tune(XCLIP_TUNE_LN_FWD_BLOCKS) > 0 && fgrid > num_sms() * tune(XCLIP_TUNE_LN_FWD_BLOCKS))
-    fgrid = num_sms() * tune(XCLIP_TUNE_LN_FWD_BLOCKS);
-  DISPATCH_NARROW(ln_fwd_kernel, d, fgrid, s, (const bf16*)x, ldx, g, (const bf16*)res,
+  DISPATCH_NARROW(ln_fwd_kernel, d, row_grid(rows), s, (const bf16*)x, ldx, g, (const bf16*)res,
                   ldres, (bf16*)out, ldo, stats, g2, (bf16*)out2, ldo2, stats2, rows, eps)
   XCLIP_LAUNCH_CHECK("ln_fwd_kernel");
   return XCLIP_OK;
@@ -685,45 +528,11 @@ extern "C" int xclip_layernorm_bwd(const void* dy, int64_t lddy, const void* x, 
                     (!add || ALIGNED16(add)),
                 "layernorm_bwd: pointers must be 16-byte aligned");
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const int per_sm = tune(XCLIP_TUNE_LN_BWD_BLOCKS) > 0 ? tune(XCLIP_TUNE_LN_BWD_BLOCKS) : 2;
+  const int per_sm = 2;
   const int grid = row_grid(rows) < num_sms() * per_sm ? row_grid(rows) : num_sms() * per_sm;
   DISPATCH_NARROW(ln_bwd_kernel, d, grid, s, (const bf16*)dy, lddy, (const bf16*)x, ldx, stats, g,
                   (const bf16*)add, ldadd, (bf16*)dx, lddx, dg, rows)
   XCLIP_LAUNCH_CHECK("ln_bwd_kernel");
-  return XCLIP_OK;
-}
-
-extern "C" int xclip_geglu_ln_fwd(const void* u, int64_t ldu, const float* g, void* h, int64_t ldh,
-                                  float* stats, int rows, int dh, float eps,
-                                  xclip_stream_t stream) {
-  int rc = xclip_init();
-  if (rc) return rc;
-  XCLIP_REQUIRE(u && g && h && stats, "geglu_ln_fwd: null pointer");
-  XCLIP_REQUIRE(rows > 0 && dh % 1024 == 0, "geglu_ln_fwd: rows=%d dh=%d (dh %% 1024)", rows, dh);
-  XCLIP_REQUIRE(ldu % 8 == 0 && ldh % 8 == 0 && ldu >= 2 * dh, "geglu_ln_fwd: bad leading dims");
-  XCLIP_REQUIRE(ALIGNED16(u) && ALIGNED16(h) && ALIGNED16(g), "geglu_ln_fwd: misaligned pointer");
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  DISPATCH_WIDE(geglu_ln_fwd_kernel, dh, wide_grid(rows, dh), s, (const bf16*)u, ldu, g, (bf16*)h, ldh,
-                stats, rows, eps)
-  XCLIP_LAUNCH_CHECK("geglu_ln_fwd_kernel");
-  return XCLIP_OK;
-}
-
-extern "C" int xclip_geglu_ln_bwd(const void* dh_, int64_t lddh, const void* u, int64_t ldu,
-                                  const float* stats, const float* g, void* du, int64_t lddu,
-                                  float* dg, int rows, int dh, xclip_stream_t stream) {
-  int rc = xclip_init();
-  if (rc) return rc;
-  XCLIP_REQUIRE(dh_ && u && stats && g && du, "geglu_ln_bwd: null pointer");
-  XCLIP_REQUIRE(rows > 0 && dh % 1024 == 0, "geglu_ln_bwd: rows=%d dh=%d (dh %% 1024)", rows, dh);
-  XCLIP_REQUIRE(lddh % 8 == 0 && ldu % 8 == 0 && lddu % 8 == 0 && ldu >= 2 * dh && lddu >= 2 * dh,
-                "geglu_ln_bwd: bad leading dims");
-  XCLIP_REQUIRE(ALIGNED16(dh_) && ALIGNED16(u) && ALIGNED16(du) && ALIGNED16(g),
-                "geglu_ln_bwd: misaligned pointer");
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  DISPATCH_WIDE(geglu_ln_bwd_kernel, dh, wide_grid(rows, dh), s, (const bf16*)dh_, lddh, (const bf16*)u, ldu,
-                stats, g, (bf16*)du, lddu, dg, rows)
-  XCLIP_LAUNCH_CHECK("geglu_ln_bwd_kernel");
   return XCLIP_OK;
 }
 

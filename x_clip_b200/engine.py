@@ -23,10 +23,6 @@ BF16 = torch.bfloat16
 F32 = torch.float32
 LN_EPS = 1e-5   # the reference's fp32 branch (x_clip.py:118); parameters/outputs are fp32-facing
 
-# Fused feed-forward (csrc/ff.cu): GEGLU in the up-projection's epilogue, LayerNorm(4d) folded into
-# the down-projection.  False selects the separate geglu_ln_fwd kernel (kept for A/B measurements).
-FUSED_FF = True
-
 _scope_cache = None     # dict while a weight_scope() is active, else None
 
 
@@ -87,49 +83,11 @@ class weight_scope:
         return False
 
 
-def clear_weight_cache() -> None:
-    """Kept for API compatibility: there is no persistent cache any more."""
-
-
 def _wgrad(dy: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
     """dW[out,in] = dy^T @ x in fp32: both operands consumed MN-major, split-K + atomics."""
     out = torch.zeros((dy.shape[1], x.shape[1]), device=dy.device, dtype=F32)
     K.gemm(dy, x, a_major=1, b_major=1, out=out, accumulate=True)
     return out
-
-
-# Weight gradients are off the critical path of the backward chain (nothing downstream reads
-# them), so the transformer backward launches them on a side stream: the tensor-bound wgrad GEMM
-# then overlaps with the HBM-bound LayerNorm / GEGLU backward kernels of the main stream (those
-# need < 3 KB of shared memory and co-reside with the persistent GEMM CTAs).
-OVERLAP_WGRAD = False   # measured neutral at cfg2 (82.9 vs 82.5 ms): the persistent GEMM leaves no room to co-schedule
-_side_streams = {}
-
-
-class _WgradStream:
-    def __init__(self, device: torch.device):
-        self.enabled = OVERLAP_WGRAD
-        self.main = torch.cuda.current_stream(device)
-        if self.enabled:
-            key = (device.index, self.main.cuda_stream)
-            if key not in _side_streams:
-                _side_streams[key] = torch.cuda.Stream(device=device)
-            self.side = _side_streams[key]
-
-    def wgrad(self, dy: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
-        if not self.enabled:
-            return _wgrad(dy, x)
-        out = torch.zeros((dy.shape[1], x.shape[1]), device=dy.device, dtype=F32)
-        self.side.wait_stream(self.main)          # operands (and the zero fill) are ready
-        with torch.cuda.stream(self.side):
-            K.gemm(dy, x, a_major=1, b_major=1, out=out, accumulate=True)
-        for t in (dy, x, out):                    # keep the allocator from recycling them early
-            t.record_stream(self.side)
-        return out
-
-    def join(self) -> None:
-        if self.enabled:
-            self.main.wait_stream(self.side)
 
 
 # Set by the micro-batched step for every chunk but the last one it back-propagates: transformer
@@ -138,7 +96,9 @@ class _WgradStream:
 # no zero-filled temporary, no `grad += new` pass per parameter and chunk.  The last chunk returns
 # ordinary gradient tensors, so post-accumulate hooks (GradSync) fire exactly once per step.
 _accumulate_into_grad = False
-INPLACE_GRAD_ACCUMULATION = True     # module switch for A/B measurements (tools/ab_step.py)
+# User option (INTEGRATION.md §3): False sends every chunk's gradients through autograd, so gradient
+# hooks fire once per chunk instead of once per step.
+INPLACE_GRAD_ACCUMULATION = True
 
 
 def _grad_target(param: torch.Tensor):
@@ -178,11 +138,11 @@ class TransformerFn(torch.autograd.Function):
         # needs_input_grad ignores no_grad): in the first sweep of the micro-batched step and in
         # inference nothing is kept for a backward, and the 8d-wide u = [value | gate] is not written
         # bf16 MMA operands of this call's weights; backward reuses exactly these (ctx.wb)
-        wb = [tuple(weight_bf16(w) for w in (l[1], l[2], l[5], l[7])) for l in layers]
+        wb = [tuple(weight_bf16(w) for w in (l[1], l[2], l[5])) for l in layers]
         # norm_in fused with the first pre-norm
         xcur, st_in, xn, st1 = K.layernorm_fwd(x_in, g_in, g2=layers[0][0], eps=LN_EPS)
         for L, (g1, wqkv, wo, go, g2, w1, g4, w2) in enumerate(layers):
-            bqkv, bo, b1, b2 = wb[L]
+            bqkv, bo, b1 = wb[L]
             qkv = K.gemm(xn, bqkv)
             if rot_cos is not None:
                 K.rotary_(qkv, n, 3 * heads, rot_cos, rot_sin)
@@ -190,18 +150,13 @@ class TransformerFn(torch.autograd.Function):
             y = K.gemm(o, bo)
             # x1 = LN(y)*go + x ; xn2 = LN(x1)*g2   (attention tail + feed-forward pre-norm)
             x1, st_y, xn2, st_x1 = K.layernorm_fwd(y, go, res=xcur, g2=g2, eps=LN_EPS)
-            if FUSED_FF:
-                # h below is hp = value*gelu(gate) BEFORE the LayerNorm (the norm is folded into
-                # the down-projection); the backward knows from ctx.fused_ff
-                w1p, w2g, colvec = ff_weights(w1, w2, g4)
-                u, h, rowsum = K.ff_up(xn2, w1p, need_u=need_bwd)
-                x2, acc, st_v = K.ff_down(h, w2g, colvec, rowsum, x1, LN_EPS)
-                if need_bwd:
-                    ff_saved.append((w2g, colvec, acc))
-            else:
-                u = K.gemm(xn2, b1)
-                h, st_v = K.geglu_ln_fwd(u, g4, eps=LN_EPS)
-                x2 = K.gemm(h, b2, residual=x1)
+            # h below is hp = value*gelu(gate) BEFORE the LayerNorm (the norm is folded into the
+            # down-projection)
+            w1p, w2g, colvec = ff_weights(w1, w2, g4)
+            u, h, rowsum = K.ff_up(xn2, w1p, need_u=need_bwd)
+            x2, acc, st_v = K.ff_down(h, w2g, colvec, rowsum, x1, LN_EPS)
+            if need_bwd:
+                ff_saved.append((w2g, colvec, acc))
             # forward-only sweeps keep NOTHING alive beyond the layer (the list below would otherwise hold
             # every layer's activations until the call returns: ~14 of the 22 d per token-layer)
             if need_bwd:
@@ -217,7 +172,6 @@ class TransformerFn(torch.autograd.Function):
         ctx.mask = mask_c
         ctx.dims = (B, n, d, heads, depth, scale, causal)
         ctx.rot = (rot_cos, rot_sin)
-        ctx.fused_ff = FUSED_FF
         ctx.ff_saved = ff_saved
         ctx.weights = weights
         ctx.wb = wb
@@ -239,7 +193,6 @@ class TransformerFn(torch.autograd.Function):
         dout = dout.contiguous()
 
         grads: List[Optional[torch.Tensor]] = [None] * len(weights)
-        wg = _WgradStream(dev)
 
         def gain_grad(idx):
             """fp32 accumulator for the gain gradient of weights[idx]: its .grad (in-place mode) or zeros"""
@@ -254,7 +207,7 @@ class TransformerFn(torch.autograd.Function):
             if tgt is not None:
                 K.gemm(dy_, x_, a_major=1, b_major=1, out=tgt, accumulate=True)
                 return None
-            return wg.wgrad(dy_, x_)
+            return _wgrad(dy_, x_)
 
         dg_out, grads[1] = gain_grad(1)
         dx = K.layernorm_bwd(dout, x_last, st_out, g_out, dg=dg_out)
@@ -262,29 +215,22 @@ class TransformerFn(torch.autograd.Function):
             g1, wqkv, wo, go, g2, w1, g4, w2 = layers[L]
             xcur, st1, xn, qkv, o, lse, y, st_y, x1, st_x1, xn2, u, st_v, h = ctx.saved[L]
             ctx.saved[L] = None
-            bqkv, bo, b1, b2 = ctx.wb[L]
+            bqkv, bo, b1 = ctx.wb[L]
             base = 2 + 8 * L
             # feed-forward: x2 = h @ w2^T + x1
             dg4, grads[base + 6] = gain_grad(base + 6)
-            if ctx.fused_ff:
-                # h is the pre-norm hp.  Row means of the LayerNorm backward from d-wide data, the
-                # LN + GEGLU backward inside the dgrad GEMM, dW2 / dg4 from dW2g = dxs^T hp - vsum
-                w2g, colvec, acc = ctx.ff_saved[L]
-                ctx.ff_saved[L] = None
-                dxs, vsum, ab = K.ff_bwd_prep(dx, st_v, acc, colvec)
-                du = K.ff_bwd(dx, w2g, u, st_v, ab)
-                dw2 = K.ff_w2_grad_post_(wg.wgrad(dxs, h), vsum, g4.detach(), w2.detach(), dg4)
-                tgt = _grad_target(w2)
-                if tgt is not None:
-                    tgt.add_(dw2)
-                    dw2 = None
-                grads[base + 7] = dw2
-                dh = None
-            else:
-                dh = K.gemm(dx, b2, b_major=1)
-                grads[base + 7] = weight_grad(base + 7, dx, h)
-                du = K.geglu_ln_bwd(dh, u, st_v, g4, dg=dg4)
-            del dh
+            # h is the pre-norm hp.  Row means of the LayerNorm backward from d-wide data, the
+            # LN + GEGLU backward inside the dgrad GEMM, dW2 / dg4 from dW2g = dxs^T hp - vsum
+            w2g, colvec, acc = ctx.ff_saved[L]
+            ctx.ff_saved[L] = None
+            dxs, vsum, ab = K.ff_bwd_prep(dx, st_v, acc, colvec)
+            du = K.ff_bwd(dx, w2g, u, st_v, ab)
+            dw2 = K.ff_w2_grad_post_(_wgrad(dxs, h), vsum, g4.detach(), w2.detach(), dg4)
+            tgt = _grad_target(w2)
+            if tgt is not None:
+                tgt.add_(dw2)
+                dw2 = None
+            grads[base + 7] = dw2
             dxn2 = K.gemm(du, b1, b_major=1)
             grads[base + 5] = weight_grad(base + 5, du, xn2)
             del du
@@ -304,7 +250,6 @@ class TransformerFn(torch.autograd.Function):
             dx = K.layernorm_bwd(dxn, xcur, st1, g1, add=dx1, dg=dg1)
         dg_in, grads[0] = gain_grad(0)
         dx_in = K.layernorm_bwd(dx, x_in, st_in, g_in, dg=dg_in)
-        wg.join()
         ctx.saved = ctx.wb = None
         return (dx_in.view(B, n, d), None, None, None, None, None, None, None, *grads)
 

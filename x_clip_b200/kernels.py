@@ -183,27 +183,6 @@ def layernorm_bwd(dy, x, stats, g, *, add=None, dg=None):
     return dx
 
 
-def geglu_ln_fwd(u, g, *, eps=1e-5):
-    _need(u, BF16, "u"); _rows2d(u, "u"); _need(g, F32, "g")
-    rows, two_dh = u.shape
-    dh = two_dh // 2
-    h = torch.empty((rows, dh), device=u.device, dtype=BF16)
-    stats = torch.empty((rows, 2), device=u.device, dtype=F32)
-    _call(u, "geglu_ln_fwd", 0.0, 2.0 * rows * dh * 3, "xclip_geglu_ln_fwd", u.data_ptr(), u.stride(0), g.data_ptr(), h.data_ptr(),
-              h.stride(0), stats.data_ptr(), rows, dh, float(eps))
-    return h, stats
-
-
-def geglu_ln_bwd(dh_grad, u, stats, g, *, dg=None):
-    _need(dh_grad, BF16, "dh"); _rows2d(dh_grad, "dh"); _need(u, BF16, "u")
-    rows, two_dh = u.shape
-    du = torch.empty((rows, two_dh), device=u.device, dtype=BF16)
-    _call(dh_grad, "geglu_ln_bwd", 0.0, 2.0 * rows * (two_dh // 2) * 5, "xclip_geglu_ln_bwd", dh_grad.data_ptr(), dh_grad.stride(0), u.data_ptr(),
-              u.stride(0), stats.data_ptr(), g.data_ptr(), du.data_ptr(), du.stride(0), _ptr(dg),
-              rows, two_dh // 2)
-    return du
-
-
 def l2norm_fwd(p):
     _need(p, F32, "p"); _rows2d(p, "p")
     rows, d = p.shape
